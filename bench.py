@@ -10,6 +10,8 @@ snapshot epoch (SURVEY.md §8d).  Reported on one JSON line:
   cpu_baseline  the oracle (C++ restatement of the reference's Java path; the JVM cannot run here) on the host cores
 `--impl reference` times only that CPU path.  N > 1 (torchrun): the registry is sharded by model across ranks (each rank
 places its slice against a replicated instance table; no data-path collective), so total work is fixed: "strong".
+`--dump-outputs DIR` writes what the last timed step computed as .npy files; the inputs are seeded, so two builds can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -34,6 +36,31 @@ SEED = {"C2": 2, "C3": 3, "C4": 4, "C5": 5}.get(CONFIG, 3)
 METRIC = "placement decisions/sec at 1M models x 10k instances"
 WORKLOADS = {"C2": "Zipf request rates, no type constraints", "C3": "mixed type constraints",
              "C5": "adversarial 95%-full capacity bin-packing, heavy type-constraint masks", "C4": "churn"}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dump_dir, arrays: dict, rank: int = 0, world: int = 1):
+    """--dump-outputs: every field of every structured array as <array>_<field>.npy in float64 (int64 values past 2**53
+    round), so that two builds can be compared output for output on the same seeded inputs.  When all of it would exceed
+    DUMP_LIMIT_BYTES, every array is cut to a fixed, seeded sample of its rows (<array>_index.npy holds the row numbers).
+    With several ranks each writes its own slice under rank<r>/."""
+    if not dump_dir:
+        return
+    if world > 1:
+        dump_dir = os.path.join(dump_dir, f"rank{rank}")
+    os.makedirs(dump_dir, exist_ok=True)
+    full = sum(len(a) * len(a.dtype.names) * 8 for a in arrays.values())
+    frac = 1.0 if full <= DUMP_LIMIT_BYTES else \
+        DUMP_LIMIT_BYTES / sum(len(a) * (len(a.dtype.names) + 1) * 8 for a in arrays.values())
+    for name, a in arrays.items():
+        if frac < 1.0:
+            idx = np.sort(np.random.default_rng(12345).choice(len(a), int(len(a) * frac), replace=False))
+            np.save(os.path.join(dump_dir, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        for f in a.dtype.names:
+            np.save(os.path.join(dump_dir, f"{name}_{f}.npy"), np.ascontiguousarray(a[f], dtype=np.float64))
 
 
 def bytes_per_decision(row_words: int) -> int:
@@ -202,10 +229,11 @@ def run_reference(args, rank: int, world: int):
     times, dense_times = [], []
     for step in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        oracle.get_next_batch(od, fl.type_names, off, idx, fl.now_ms, SEED, threads=threads)
+        res = oracle.get_next_batch(od, fl.type_names, off, idx, fl.now_ms, SEED, threads=threads)
         dt = time.perf_counter() - t0
         if step >= args.warmup:
             times.append(dt)
+    dump_outputs(args.dump_outputs, {"decision": res[["target", "n_candidates"]]})
     for step in range(min(3, args.steps)):
         t0 = time.perf_counter()
         oracle.get_next_batch(od, fl.type_names, off, idx, fl.now_ms, SEED, threads=threads, dense=True)
@@ -282,9 +310,10 @@ def run_reference_churn(args):
         ev = w.events(ep, CHURN_EVENTS, SEED)
         now0 = fl.now_ms + ep * w.window_ms
         t0 = time.perf_counter()
-        sim.step(ev, now0, now0 + w.window_ms, 400 + ep)
+        dec, evi, rows, _, _ = sim.step(ev, now0, now0 + w.window_ms, 400 + ep)
         if ep >= args.warmup:
             times.append(time.perf_counter() - t0)
+    dump_outputs(args.dump_outputs, {"decision": dec, "eviction": evi, "instance": rows})
     value = CHURN_EVENTS * len(times) / sum(times)
     print(json.dumps({
         "impl": "reference", "metric": CHURN_METRIC, "value": value, "unit": "events/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -356,6 +385,7 @@ def run_churn(args, rank: int, world: int, local_rank: int):
             n_dec += len(dec); n_evict += len(evi); n_lru += rep.n_lru_events; n_pub += rep.n_published
     clocks = sampler.finish()
     launches = s.kernel_launches() - launches0
+    dump_outputs(args.dump_outputs, {"decision": dec, "eviction": evi, "instance": rows})
     ph = np.asarray(phases)
     k = len(dev_ms)
     # standalone commits through the C ABI: a window's worth of numeric instance updates -> device path; one string change -> structural
@@ -425,7 +455,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-instance-shards", action="store_true", help="N > 1: skip the instance-sharded leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -497,6 +530,7 @@ def main():
     dev_ms = float(np.sum(kernel_ms))
     out_dev = np.zeros(B, dtype=DECISION_OUT)
     solver._ck(lib.mmp_device_download(solver.h, out_dev.ctypes.data_as(C.c_void_p), d_out, out_dev.nbytes))
+    dump_outputs(args.dump_outputs, {"decision": out_dev}, rank, world)
 
     # ---- end to end through the C ABI with pinned host buffers ----
     e2e_ms = []
@@ -789,5 +823,6 @@ def _only_the_json_line_on_stdout():
 OUT = sys.stdout
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (which may be read-only)
     _only_the_json_line_on_stdout()
     main()

@@ -3,8 +3,9 @@
 every decision routine of the product (decide_stream with full and tiny windows/budgets, decide_fast 32/16, budgeted
 single-lane decide_ctx) against the oracle on 600 mixed decisions each, and the instance-shard min-loc protocol (2/3/5/8
 shards) against the unsharded result.  usage: random_sweep.py LO HI"""
-import sys, ctypes as C, numpy as np, time
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+import os, sys, ctypes as C, numpy as np, time
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 from modelmesh_b200 import _lib
 from modelmesh_b200.fleet import Fleet
 from modelmesh_b200.sharding import combine_shard_keys, decode_shard_keys
@@ -12,7 +13,7 @@ from modelmesh_b200.synth import make_decisions, make_fleet, load_into_fleet
 from helpers import oracle_from_synth, solver_from_synth, compare_decisions
 from oracle import binding
 binding.build()
-lib = _lib.load("/root/repo/tests/emul/_build/libmmplace_emul.so", require_all=False)
+lib = _lib.load(os.path.join(ROOT, "tests", "emul", "_build", "libmmplace_emul.so"), require_all=False)
 lib.mmp_emul_set_keys.argtypes = [C.c_void_p, C.c_void_p]
 lib.mmp_emul_lane_bails.restype = C.c_long
 t0 = time.time(); bad = 0; n_dec = 0
